@@ -11,6 +11,13 @@ the same default run covers the rest of the metric ("@64^2 & 256^2"): `sample` =
 `train_256` = configs[2] (EDM UNet 256^2 with self-attention, B = 64 per GPU = 512 over 8 GPUs),
 `sample_256_heun` = configs[4] (Heun 18/50/100 steps, B = 32 per GPU, replicas), `sample_256_text_cfg` =
 configs[3] (text cross-attention, CFG Euler-ancestral 30 steps, B = 64).  Prints ONE JSON line.
+Every timed training loop runs --steps steps.
+
+    python bench.py ... --dump-outputs DIR   # also write what the timed path computed as DIR/<name>.npy
+
+The inputs are seeded, so two builds run with the same arguments can be compared output for output: per training
+workload the loss, parameters, EMA parameters and Adam moments after the last timed step; per sampler run the
+images it returned.
 """
 from __future__ import annotations
 
@@ -87,6 +94,33 @@ def emit(obj) -> None:
     out = _JSON_OUT if _JSON_OUT is not None else sys.stdout
     out.write(json.dumps(obj) + "\n")
     out.flush()
+
+
+_OUTPUTS = None                 # name -> float32 host array, collected on rank 0 when --dump-outputs is given
+OUTPUT_MAX_ELEMS = 1 << 20      # per array; 13 arrays in the default run stay under OUTPUT_MAX_BYTES
+OUTPUT_MAX_BYTES = 64 << 20
+
+
+def keep_output(name: str, t) -> None:
+    """Record `t` for --dump-outputs as a float32 host copy; above OUTPUT_MAX_ELEMS elements, a sample at
+    fixed seeded indices (the same indices in every run for the same size)."""
+    if _OUTPUTS is None:
+        return
+    import numpy as np
+    a = t.detach().float().cpu().numpy()
+    if a.size > OUTPUT_MAX_ELEMS:
+        a = a.reshape(-1)[np.sort(np.random.default_rng(0).integers(0, a.size, OUTPUT_MAX_ELEMS))]
+    _OUTPUTS[name] = a
+
+
+def write_outputs(directory: str) -> None:
+    import numpy as np
+    total = sum(a.nbytes for a in _OUTPUTS.values())
+    if total > OUTPUT_MAX_BYTES:
+        raise RuntimeError(f"--dump-outputs: {total} bytes exceed the {OUTPUT_MAX_BYTES}-byte limit")
+    os.makedirs(directory, exist_ok=True)
+    for name, a in _OUTPUTS.items():
+        np.save(os.path.join(directory, name + ".npy"), a)
 
 
 def roofline_traffic(workload: str, batch: int) -> dict:
@@ -446,6 +480,10 @@ def run_train(D, args, workload, steps, warmup, with_cpu_baseline):
     e3.record()
     D.sync()
     clk = clocks.stop()
+    st = trainer.state
+    for name, t in (("loss", loss), ("params", st.params.flat), ("ema_params", st.ema_params.flat),
+                    ("adam_mu", st.opt_state["mu"]), ("adam_nu", st.opt_state["nu"])):
+        keep_output(f"{workload}_train_{name}", t)
     ms_e2e = e2.elapsed_time(e3) / steps
     ms_dev, ms_e2e = D.max_ms(ms_dev, ms_e2e)
     log(f'{workload}: {ms_dev:.2f} ms/step device, {ms_e2e:.2f} e2e')
@@ -524,6 +562,7 @@ def run_euler_c2(D, args, trainer, model, workload="c2"):
     imgs = sampler.generate_samples(params, B, res, diffusion_steps=n_s, start_step=1000, device=dev)
     s1.record()
     D.sync()
+    keep_output(f"{workload}_sample{n_s}_images", imgs)
     (ms_s,) = D.max_ms(s0.elapsed_time(s1))
     return {"sampler": "EulerSampler", "diffusion_steps": n_s, "batch_per_gpu": B,
             "denoise_steps_per_sec": n_s / (ms_s / 1e3), "image_steps_per_sec": world * B * n_s / (ms_s / 1e3),
@@ -579,6 +618,7 @@ def sampling_runs(D, args, workload):
                                     model_conditioning_inputs=cond)
         s1.record()
         D.sync()
+        keep_output(f"{workload}_sample{n}_images", img)
         (ms,) = D.max_ms(s0.elapsed_time(s1))
         runs.append({"diffusion_steps": n, "unet_evals_per_image": nfe, "ms": ms,
                      "denoise_steps_per_sec": n / (ms / 1e3), "image_steps_per_sec": world * B * n / (ms / 1e3),
@@ -591,6 +631,7 @@ def sampling_runs(D, args, workload):
 
 
 def main():
+    global _OUTPUTS
     claim_stdout()
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -608,7 +649,13 @@ def main():
     ap.add_argument("--no-graph", action="store_true")
     ap.add_argument("--ref-batch", type=int, default=16)
     ap.add_argument("--ref-max-steps", type=int, default=3)
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the timed path computed in its last step as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "fdx":
+        ap.error("--dump-outputs records the fdx path only")
     import faulthandler
     faulthandler.enable()
     if os.environ.get("FDX_BENCH_WATCHDOG"):
@@ -623,6 +670,8 @@ def main():
     import torch
     D = Dist()
     hbm, tf_burst, tf_sust, src = load_peaks()
+    if args.dump_outputs and D.rank == 0:
+        _OUTPUTS = {}
 
     if args.workload in ("c4", "c5"):
         blk = sampling_runs(D, args, args.workload)
@@ -640,6 +689,8 @@ def main():
                                "achieved": head["tensor_frac_of_sustained"] * tf_sust, "peak": tf_sust,
                                "unit": "TFLOP/s", "frac": head["tensor_frac_of_sustained"],
                                "peak_source": f"{src} bf16_tflops_sustained", "traffic": None}})
+            if _OUTPUTS is not None:
+                write_outputs(args.dump_outputs)
         return D.close()
 
     first = "c2" if args.workload == "all" else args.workload
@@ -654,13 +705,12 @@ def main():
     if args.workload == "all" and not args.no_256:
         # the 256x256 half of the metric: C3 training (B = 64 per GPU: global 512 at --gpus 8 = BASELINE
         # configs[2]), C5 Heun sweep and C4 CFG sampling as per-GPU replicas
-        steps256 = max(5, args.steps // 4)
-        b3, tr3, m3 = run_train(D, args, "c3", steps256, 3, with_cpu_baseline=False)
+        b3, tr3, m3 = run_train(D, args, "c3", args.steps, 3, with_cpu_baseline=False)
         del tr3, m3
         gc.collect()
         torch.cuda.empty_cache()
         if b3 is not None:
-            b3.update({"metric": "train_images_per_sec", "unit": "images/s", "steps": steps256, "warmup": 3})
+            b3.update({"metric": "train_images_per_sec", "unit": "images/s", "steps": args.steps, "warmup": 3})
         extra["train_256"] = b3
         if not args.no_sample:
             extra["sample_256_heun"] = sampling_runs(D, args, "c5")
@@ -676,6 +726,8 @@ def main():
         out["sample"] = sample
         out.update(extra)
         emit(out)
+        if _OUTPUTS is not None:
+            write_outputs(args.dump_outputs)
     D.close()
 
 
