@@ -6,5 +6,3 @@ arithmetic runs in the hand-written CUDA kernels of libfdx.so (include/fdx.h).  
 CPU or eager fallback: ops raise if the library is missing or tensors are not on a GPU.
 """
 __version__ = "0.1.0"
-
-from . import _defaults  # noqa: E402,F401  (kernel-generation defaults -> environment, before libfdx loads)

@@ -11,7 +11,6 @@
 // fully coalesced; per-(image,group) partial sums are reduced with warp shuffles,
 // then shared-memory atomics, then one global atomic per block.
 #include "fdx_common.cuh"
-#include <stdlib.h>
 #include "../../include/fdx.h"
 
 namespace {
@@ -191,26 +190,25 @@ __device__ __forceinline__ f32x2_t gn_dz_pair(f32x2_t x, f32x2_t dy, f32x2_t ah,
   return f2_mul(dy, f2_mul(s, u));
 }
 
-// red != nullptr: the finalize step is MERGED into this kernel - both of its outputs are linear in the
-// per-(image, channel) sums, so every CTA adds its partial's contribution straight into red[n][g][2] (zeroed by
-// the caller), dgamma[c] and dbeta[c], and zeroes the column-sum outputs the second pass accumulates into.
-// One launch (and one dependent-launch gap) less on the backward's critical path per GroupNorm.
+// Pass 1 with the finalize step merged in: both of its outputs are linear in the per-(image, channel) sums,
+// so every CTA adds its partial's contribution straight into red[n][g][2] (zeroed by the caller), dgamma[c]
+// and dbeta[c], and zeroes the column-sum outputs the second pass accumulates into.
 template <bool SILU>
 __global__ void __launch_bounds__(kNT, 3)
 gn_bwd_stats_kernel(const __nv_bfloat16* __restrict__ x, long long xps,
                     const __nv_bfloat16* __restrict__ dy, long long dps, int HW, int C, int G,
                     const float* __restrict__ stats, const float* __restrict__ gamma,
-                    const float* __restrict__ beta, float eps, float* __restrict__ ws,
+                    const float* __restrict__ beta, float eps,
                     float* __restrict__ red, float* __restrict__ dgamma, float* __restrict__ dbeta,
                     float* __restrict__ csum_img, float* __restrict__ csum_tot) {
   const int vpp = C >> 3, rows = kNT / vpp, cpg = C / G;
   const int n = blockIdx.y;
   const int tid = threadIdx.x;
-  extern __shared__ float shm[];   // 2 * [rows*C] (+ 2 * C with the merged finalize)
+  extern __shared__ float shm[];   // 2 * [rows*C] + 2 * [C]
   float* part0 = shm;
   float* part1 = part0 + rows * C;
   const float cnt = (float)HW * (float)cpg;
-  if (red && blockIdx.x == 0) {
+  if (blockIdx.x == 0) {
     if (csum_img) for (int c = tid; c < C; c += kNT) csum_img[(long long)n * C + c] = 0.f;
     if (csum_tot && n == 0) for (int c = tid; c < C; c += kNT) csum_tot[c] = 0.f;
   }
@@ -268,100 +266,27 @@ gn_bwd_stats_kernel(const __nv_bfloat16* __restrict__ x, long long xps,
     }
   }
   __syncthreads();
-  if (red) {
-    float* gr0 = part1 + rows * C;   // [C] gamma_c * S0,  [C] gamma_c * rstd * (S1 - mean * S0)
-    float* gr1 = gr0 + C;
-    for (int c = tid; c < C; c += kNT) {
-      float t0 = 0.f, t1 = 0.f;
-      for (int rr = 0; rr < rows; ++rr) { t0 += part0[rr * C + c]; t1 += part1[rr * C + c]; }
-      const int g = c / cpg;
-      const float mean = stats[(long long)n * 2 * G + 2 * g] / cnt;
-      const float var = fmaxf(0.f, stats[(long long)n * 2 * G + 2 * g + 1] / cnt - mean * mean);
-      const float u = rsqrtf(var + eps) * (t1 - mean * t0);
-      atomicAdd(&dbeta[c], t0);
-      atomicAdd(&dgamma[c], u);
-      const float ga = gamma[c];
-      gr0[c] = ga * t0;
-      gr1[c] = ga * u;
-    }
-    __syncthreads();
-    for (int g = tid; g < G; g += kNT) {
-      float r0 = 0.f, r1 = 0.f;
-      for (int c = g * cpg; c < (g + 1) * cpg; ++c) { r0 += gr0[c]; r1 += gr1[c]; }
-      atomicAdd(&red[(long long)n * 2 * G + 2 * g], r0);
-      atomicAdd(&red[(long long)n * 2 * G + 2 * g + 1], r1);
-    }
-    return;
-  }
-  // per-(image, channel) partial sums: only gridDim.x (<= ~10) atomics ever hit one address
+  float* gr0 = part1 + rows * C;   // [C] gamma_c * S0,  [C] gamma_c * rstd * (S1 - mean * S0)
+  float* gr1 = gr0 + C;
   for (int c = tid; c < C; c += kNT) {
     float t0 = 0.f, t1 = 0.f;
     for (int rr = 0; rr < rows; ++rr) { t0 += part0[rr * C + c]; t1 += part1[rr * C + c]; }
-    atomicAdd(&ws[((long long)n * C + c) * 2], t0);
-    atomicAdd(&ws[((long long)n * C + c) * 2 + 1], t1);
-  }
-}
-
-// finalize: blocks [0, cb) reduce over images -> dgamma / dbeta (accumulated into the gradient
-// buffers), 8 channels x 32 image lanes per block (the image loop is a chain of dependent-latency
-// loads: 32 lanes x 4-way unrolling keeps it to one or two round trips); blocks [cb, cb + gb) reduce
-// over the channels of a group -> red[n][g], one warp per (image, group).
-constexpr int kFinC = 8;     // channels per dgamma/dbeta block
-__global__ void __launch_bounds__(256)
-gn_bwd_finalize_kernel(const float* __restrict__ ws, const float* __restrict__ stats,
-                       const float* __restrict__ gamma, int N, int HW, int C, int G, float eps, int cb,
-                       float* __restrict__ red, float* __restrict__ dgamma, float* __restrict__ dbeta) {
-  const int cpg = C / G;
-  const float cnt = (float)HW * (float)cpg;
-  __shared__ float sh0[32][kFinC + 1], sh1[32][kFinC + 1];
-  if ((int)blockIdx.x < cb) {
-    const int cl = threadIdx.x % kFinC, nl = threadIdx.x / kFinC;
-    const int c = blockIdx.x * kFinC + cl;
-    float a0 = 0.f, a1 = 0.f;
-    if (c < C) {
-      const int g = c / cpg;
-#pragma unroll 4
-      for (int n = nl; n < N; n += 32) {
-        const float2 st = *reinterpret_cast<const float2*>(stats + (long long)n * 2 * G + 2 * g);
-        const float2 s = *reinterpret_cast<const float2*>(ws + ((long long)n * C + c) * 2);
-        const float mean = st.x / cnt;
-        const float var = fmaxf(0.f, st.y / cnt - mean * mean);
-        const float rstd = rsqrtf(var + eps);
-        a0 += s.x;
-        a1 += rstd * (s.y - mean * s.x);
-      }
-    }
-    sh0[nl][cl] = a0;
-    sh1[nl][cl] = a1;
-    __syncthreads();
-    if (nl == 0 && c < C) {
-      float t0 = 0.f, t1 = 0.f;
-#pragma unroll
-      for (int k = 0; k < 32; ++k) { t0 += sh0[k][cl]; t1 += sh1[k][cl]; }
-      dbeta[c] += t0;
-      dgamma[c] += t1;
-    }
-  } else {
-    const int i = (blockIdx.x - cb) * 8 + (threadIdx.x >> 5);     // (n, g), one warp each
-    if (i >= N * G) return;
-    const int lane = threadIdx.x & 31;
-    const int n = i / G, g = i % G;
+    const int g = c / cpg;
     const float mean = stats[(long long)n * 2 * G + 2 * g] / cnt;
     const float var = fmaxf(0.f, stats[(long long)n * 2 * G + 2 * g + 1] / cnt - mean * mean);
-    const float rstd = rsqrtf(var + eps);
+    const float u = rsqrtf(var + eps) * (t1 - mean * t0);
+    atomicAdd(&dbeta[c], t0);
+    atomicAdd(&dgamma[c], u);
+    const float ga = gamma[c];
+    gr0[c] = ga * t0;
+    gr1[c] = ga * u;
+  }
+  __syncthreads();
+  for (int g = tid; g < G; g += kNT) {
     float r0 = 0.f, r1 = 0.f;
-    for (int c = g * cpg + lane; c < (g + 1) * cpg; c += 32) {
-      const float2 s = *reinterpret_cast<const float2*>(ws + ((long long)n * C + c) * 2);
-      const float ga = gamma[c];
-      r0 += ga * s.x;
-      r1 += ga * rstd * (s.y - mean * s.x);
-    }
-    r0 = warp_sum(r0);
-    r1 = warp_sum(r1);
-    if (lane == 0) {
-      red[(long long)n * 2 * G + 2 * g] = r0;
-      red[(long long)n * 2 * G + 2 * g + 1] = r1;
-    }
+    for (int c = g * cpg; c < (g + 1) * cpg; ++c) { r0 += gr0[c]; r1 += gr1[c]; }
+    atomicAdd(&red[(long long)n * 2 * G + 2 * g], r0);
+    atomicAdd(&red[(long long)n * 2 * G + 2 * g + 1], r1);
   }
 }
 
@@ -383,23 +308,6 @@ gn_coeffs_kernel(const float* __restrict__ stats, const float* __restrict__ gamm
   }
 }
 
-// sums[n][c] = (S0, S1) <- sum over slots of wsl[slot][n][{0,1}][c]   (fused-epilogue workspace layout)
-__global__ void __launch_bounds__(256)
-gn_collapse_slots_kernel(const float* __restrict__ wsl, int slots, int N, int C, float* __restrict__ sums) {
-  for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < (long long)N * C;
-       i += (long long)gridDim.x * blockDim.x) {
-    const int n = (int)(i / C), c = (int)(i % C);
-    float s0 = 0.f, s1 = 0.f;
-    for (int sl = 0; sl < slots; ++sl) {
-      const float* b = wsl + (((long long)sl * N + n) * 2) * C + c;
-      s0 += b[0];
-      s1 += b[C];
-    }
-    sums[i * 2] = s0;
-    sums[i * 2 + 1] = s1;
-  }
-}
-
 // stats[n][g] = (sum, sumsq) from the per-(image, channel) sums a convolution epilogue accumulated:
 // cols[slot][n][{0,1}][C]; one warp per (image, group)
 __global__ void __launch_bounds__(256)
@@ -418,25 +326,6 @@ gn_stats_from_cols_kernel(const float* __restrict__ cols, int slots, int N, int 
   if (lane == 0) {
     stats[(long long)n * 2 * G + 2 * g] = s;
     stats[(long long)n * 2 * G + 2 * g + 1] = q;
-  }
-}
-
-// out[c] (+)= sum_r in[r][c]; 32 columns x 8 row lanes per block
-__global__ void __launch_bounds__(256)
-reduce_rows_kernel(const float* __restrict__ in, int R, int C, float* __restrict__ out, int accumulate) {
-  __shared__ float sh[8][33];
-  const int cl = threadIdx.x & 31, rl = threadIdx.x >> 5;
-  const int c = blockIdx.x * 32 + cl;
-  float a = 0.f;
-  if (c < C)
-    for (int r = rl; r < R; r += 8) a += in[(long long)r * C + c];
-  sh[rl][cl] = a;
-  __syncthreads();
-  if (rl == 0 && c < C) {
-    float t = 0.f;
-#pragma unroll
-    for (int k = 0; k < 8; ++k) t += sh[k][cl];
-    out[c] = accumulate ? out[c] + t : t;
   }
 }
 
@@ -571,490 +460,6 @@ gn_bwd_apply_kernel(const __nv_bfloat16* __restrict__ x, long long xps,
   }
 }
 
-// ---- GroupNorm(+SiLU) backward in ONE launch: a thread-block CLUSTER per image ------------------------
-// The two-pass backward above reads x and dy twice from HBM (8 B + 2 B written per element).  The
-// statistics it needs are per IMAGE, so here a cluster of CL CTAs owns one image: every CTA runs pass 1 on
-// its slice of the pixels, the per-channel sums are exchanged through distributed shared memory
-// (mapa + ld.shared::cluster), every CTA derives the per-group constants, and pass 2 re-reads the SAME
-// slice - a few hundred microseconds later at most, while the lines are still in the 126 MB L2 (the launch
-// keeps the images in flight, 148 / CL clusters, below ~48 MB of x + dy).  HBM traffic: 4 B read + 2 B
-// written per element.  ws[n][c] = (S0, S1) is still written (rank 0) for the dgamma / dbeta finalize.
-__device__ __forceinline__ uint32_t cluster_nctarank() {
-  uint32_t r;
-  asm volatile("mov.u32 %0, %%cluster_nctarank;" : "=r"(r));
-  return r;
-}
-__device__ __forceinline__ float ld_dsmem_f32(const float* local_ptr, uint32_t rank) {
-  uint32_t ra;
-  float v;
-  asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(ra) : "r"(smem_u32(local_ptr)), "r"(rank));
-  asm volatile("ld.shared::cluster.f32 %0, [%1];" : "=f"(v) : "r"(ra) : "memory");
-  return v;
-}
-
-template <bool SILU, bool ACC, bool CS>
-__global__ void __launch_bounds__(kNT, 2)
-gn_bwd_cluster_kernel(const __nv_bfloat16* __restrict__ x, long long xps,
-                      const __nv_bfloat16* __restrict__ dy, long long dps, int HW, int C, int G,
-                      const float* __restrict__ stats, const float* __restrict__ gamma,
-                      const float* __restrict__ beta, float eps, float* __restrict__ ws,
-                      __nv_bfloat16* __restrict__ dx, long long dxps, float* __restrict__ csum_img, const __nv_bfloat16* __restrict__ acc, long long accps) {
-  const int vpp = C >> 3, rows = kNT / vpp, cpg = C / G;
-  const uint32_t CL = cluster_nctarank(), rank = cluster_ctarank();
-  const int n = blockIdx.x / CL;
-  const int tid = threadIdx.x;
-  extern __shared__ float shm[];
-  float* part0 = shm;                      // [rows*C]   pass-1 partials / pass-2 column sums
-  float* part1 = part0 + rows * C;         // [rows*C]
-  float* tot = part1 + rows * C;           // [2*C]  this CTA's per-channel sums (read by the peers)
-  float* redg = tot + 2 * C;               // [2*G]
-  const float cnt = (float)HW * (float)cpg;
-  const int p_lo = (int)(((long long)HW * rank) / CL), p_hi = (int)(((long long)HW * (rank + 1)) / CL);
-  const bool active = tid < rows * vpp;
-  const int cv = tid % vpp, r = tid / vpp;
-  const int g = (cv * 8) / cpg;
-  float mean = 0.f, rstd = 0.f;
-  GnPair4 ah, bh;
-  const __nv_bfloat16* xb = x + (long long)n * HW * xps + cv * 8;
-  const __nv_bfloat16* db_ = dy + (long long)n * HW * dps + cv * 8;
-  if (active) {
-    mean = stats[(long long)n * 2 * G + 2 * g] / cnt;
-    const float var = fmaxf(0.f, stats[(long long)n * 2 * G + 2 * g + 1] / cnt - mean * mean);
-    rstd = rsqrtf(var + eps);
-    GnPair4 s0, s1;
-#pragma unroll
-    for (int j = 0; j < 4; ++j) {
-      const float a0 = rstd * gamma[cv * 8 + 2 * j], a1 = rstd * gamma[cv * 8 + 2 * j + 1];
-      ah.v[j] = f2_pack(0.5f * a0, 0.5f * a1);
-      bh.v[j] = SILU ? f2_pack(0.5f * (beta[cv * 8 + 2 * j] - mean * a0), 0.5f * (beta[cv * 8 + 2 * j + 1] - mean * a1))
-                     : f2_pack(0.f, 0.f);
-      s0.v[j] = f2_pack(0.f, 0.f);
-      s1.v[j] = f2_pack(0.f, 0.f);
-    }
-    for (int p0 = p_lo + r; p0 < p_hi; p0 += kBU * rows) {
-      uint4 xu[kBU], du[kBU];
-#pragma unroll
-      for (int k = 0; k < kBU; ++k) {
-        const int p = p0 + k * rows;
-        xu[k] = make_uint4(0, 0, 0, 0);
-        du[k] = make_uint4(0, 0, 0, 0);
-        if (p < p_hi) {
-          xu[k] = *reinterpret_cast<const uint4*>(xb + (long long)p * xps);
-          du[k] = *reinterpret_cast<const uint4*>(db_ + (long long)p * dps);
-        }
-      }
-#pragma unroll
-      for (int k = 0; k < kBU; ++k) {
-        const uint32_t xw[4] = {xu[k].x, xu[k].y, xu[k].z, xu[k].w};
-        const uint32_t dw[4] = {du[k].x, du[k].y, du[k].z, du[k].w};
-#pragma unroll
-        for (int j = 0; j < 4; ++j) {
-          const f32x2_t xv = f2_from_bf16x2(xw[j]);
-          const f32x2_t dz = gn_dz_pair<SILU, false>(xv, f2_from_bf16x2(dw[j]), ah.v[j], bh.v[j]);
-          s0.v[j] = f2_add(s0.v[j], dz);
-          s1.v[j] = f2_fma(dz, xv, s1.v[j]);
-        }
-      }
-    }
-#pragma unroll
-    for (int j = 0; j < 4; ++j) {
-      float lo, hi;
-      f2_unpack(s0.v[j], lo, hi);
-      part0[r * C + cv * 8 + 2 * j] = lo; part0[r * C + cv * 8 + 2 * j + 1] = hi;
-      f2_unpack(s1.v[j], lo, hi);
-      part1[r * C + cv * 8 + 2 * j] = lo; part1[r * C + cv * 8 + 2 * j + 1] = hi;
-    }
-  }
-  __syncthreads();
-  for (int c = tid; c < C; c += kNT) {
-    float t0 = 0.f, t1 = 0.f;
-    for (int rr = 0; rr < rows; ++rr) { t0 += part0[rr * C + c]; t1 += part1[rr * C + c]; }
-    tot[c] = t0;
-    tot[C + c] = t1;
-  }
-  cluster_sync_all();                       // every CTA's `tot` is complete and visible cluster-wide
-  if (tid < 2 * G) redg[tid] = 0.f;
-  __syncthreads();
-  for (int c = tid; c < C; c += kNT) {
-    float S0 = 0.f, S1 = 0.f;
-    for (uint32_t k = 0; k < CL; ++k) { S0 += ld_dsmem_f32(tot + c, k); S1 += ld_dsmem_f32(tot + C + c, k); }
-    if (rank == 0) {
-      ws[((long long)n * C + c) * 2] = S0;
-      ws[((long long)n * C + c) * 2 + 1] = S1;
-    }
-    const int gc = c / cpg;
-    const float mg = stats[(long long)n * 2 * G + 2 * gc] / cnt;
-    const float vg = fmaxf(0.f, stats[(long long)n * 2 * G + 2 * gc + 1] / cnt - mg * mg);
-    const float rg = rsqrtf(vg + eps), ga = gamma[c];
-    atomicAdd(&redg[2 * gc], ga * S0);
-    atomicAdd(&redg[2 * gc + 1], ga * rg * (S1 - mg * S0));
-  }
-  cluster_sync_all();                       // peers are done reading this CTA's `tot`; redg complete
-  // ---- pass 2 on the same pixel slice (L2-resident) ----
-  if (active) {
-    const float m1 = redg[2 * g] / cnt, m2 = redg[2 * g + 1] / cnt;
-    const float c2 = rstd * rstd * m2;
-    const float c3 = mean * c2 - rstd * m1;
-    const f32x2_t nc2 = f2_pack(-c2, -c2), c3p = f2_pack(c3, c3);
-    GnPair4 cs;
-#pragma unroll
-    for (int j = 0; j < 4; ++j) cs.v[j] = f2_pack(0.f, 0.f);
-    __nv_bfloat16* ob = dx + (long long)n * HW * dxps + cv * 8;
-    const __nv_bfloat16* ab_ = ACC ? acc + (long long)n * HW * accps + cv * 8 : nullptr;
-    for (int p0 = p_lo + r; p0 < p_hi; p0 += kBU * rows) {
-      uint4 xu[kBU], du[kBU], ou[kBU];
-#pragma unroll
-      for (int k = 0; k < kBU; ++k) {
-        const int p = p0 + k * rows;
-        xu[k] = make_uint4(0, 0, 0, 0);
-        du[k] = make_uint4(0, 0, 0, 0);
-        ou[k] = make_uint4(0, 0, 0, 0);
-        if (p < p_hi) {
-          xu[k] = *reinterpret_cast<const uint4*>(xb + (long long)p * xps);
-          du[k] = *reinterpret_cast<const uint4*>(db_ + (long long)p * dps);
-          if (ACC) ou[k] = *reinterpret_cast<const uint4*>(ab_ + (long long)p * accps);
-        }
-      }
-#pragma unroll
-      for (int k = 0; k < kBU; ++k) {
-        const int p = p0 + k * rows;
-        if (p < p_hi) {
-          const uint32_t xw[4] = {xu[k].x, xu[k].y, xu[k].z, xu[k].w};
-          const uint32_t dw[4] = {du[k].x, du[k].y, du[k].z, du[k].w};
-          const uint32_t ow[4] = {ou[k].x, ou[k].y, ou[k].z, ou[k].w};
-          uint32_t res[4];
-#pragma unroll
-          for (int j = 0; j < 4; ++j) {
-            const f32x2_t xv = f2_from_bf16x2(xw[j]);
-            const f32x2_t dz2 = gn_dz_pair<SILU, true>(xv, f2_from_bf16x2(dw[j]), ah.v[j], bh.v[j]);
-            f32x2_t v = f2_fma(dz2, ah.v[j], f2_fma(xv, nc2, c3p));
-            if (CS) cs.v[j] = f2_add(cs.v[j], v);
-            if (ACC) v = f2_add(v, f2_from_bf16x2(ow[j]));
-            res[j] = f2_to_bf16x2(v);
-          }
-          *reinterpret_cast<uint4*>(ob + (long long)p * dxps) = make_uint4(res[0], res[1], res[2], res[3]);
-        }
-      }
-    }
-    if (CS) {
-#pragma unroll
-      for (int j = 0; j < 4; ++j) {
-        float lo, hi;
-        f2_unpack(cs.v[j], lo, hi);
-        part0[r * C + cv * 8 + 2 * j] = lo;
-        part0[r * C + cv * 8 + 2 * j + 1] = hi;
-      }
-    }
-  }
-  if (CS) {
-    __syncthreads();
-    for (int c = tid; c < C; c += kNT) {
-      float v = 0.f;
-      for (int rr = 0; rr < rows; ++rr) v += part0[rr * C + c];
-      atomicAdd(&csum_img[(long long)n * C + c], v);
-    }
-  }
-}
-
-// ---- GroupNorm(+SiLU) backward as ONE persistent, software-pipelined launch (any image size) ------------
-// The cluster kernel above needs a whole image's x + dy (times the images in flight) inside the L2; a
-// 256x256x64 image alone is 16.8 MB.  Here the batch is cut into STAGES of whole images sized so that two
-// stages fit the L2 (~24 MB each).  A grid of co-resident CTAs (cooperative launch) walks the stages in
-// lock step: pass 1 of stage s (per-channel sums -> global atomics, then one release-increment of the
-// stage's arrival counter), then - after an acquire-spin on stage s-1's counter, which every CTA reaches at
-// about the same time - pass 2 of stage s-1 from L2.  One launch, x and dy read from HBM once.
-__device__ __forceinline__ unsigned ld_acquire_u32(const unsigned* p) {
-  unsigned v;
-  asm volatile("ld.acquire.gpu.global.u32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
-  return v;
-}
-
-template <bool SILU, bool ACC, bool CS>
-__global__ void __launch_bounds__(kNT, 2)
-gn_bwd_pipe_kernel(const __nv_bfloat16* __restrict__ x, long long xps, const __nv_bfloat16* __restrict__ dy,
-                   long long dps, int N, int HW, int C, int G, int imgs_per_stage,
-                   const float* __restrict__ stats, const float* __restrict__ gamma,
-                   const float* __restrict__ beta, float eps, float* __restrict__ ws,
-                   unsigned* __restrict__ counters, __nv_bfloat16* __restrict__ dx, long long dxps,
-                   float* __restrict__ csum_img, const __nv_bfloat16* __restrict__ acc, long long accps) {
-  const int vpp = C >> 3, rows = kNT / vpp, cpg = C / G;
-  const int tid = threadIdx.x;
-  extern __shared__ float shm[];
-  float* part0 = shm;                      // [rows*C]
-  float* part1 = part0 + rows * C;         // [rows*C]
-  float* redg = part1 + rows * C;          // [2*G]
-  const float cnt = (float)HW * (float)cpg;
-  const bool active = tid < rows * vpp;
-  const int cv = tid % vpp, r = tid / vpp;
-  const int g = (cv * 8) / cpg;
-  const int nstage = (N + imgs_per_stage - 1) / imgs_per_stage;
-  const unsigned nctas = gridDim.x;
-  float gam[8], bet[8];
-  if (active) {
-#pragma unroll
-    for (int j = 0; j < 8; ++j) { gam[j] = gamma[cv * 8 + j]; bet[j] = beta[cv * 8 + j]; }
-  }
-
-  // this CTA's pixel slice [lo, hi) of stage s, in the stage's flattened (image, pixel) space
-  auto slice = [&](int s, long long& lo, long long& hi, int& n0) {
-    n0 = s * imgs_per_stage;
-    const int n1 = min(N, n0 + imgs_per_stage);
-    const long long total = (long long)(n1 - n0) * HW;
-    long long per = (total + nctas - 1) / nctas;
-    per = (per + rows - 1) / rows * rows;
-    lo = min(total, (long long)blockIdx.x * per);
-    hi = min(total, lo + per);
-  };
-  auto coeffs = [&](int n, float& mean, float& rstd, GnPair4& ah, GnPair4& bh) {
-    mean = stats[(long long)n * 2 * G + 2 * g] / cnt;
-    const float var = fmaxf(0.f, stats[(long long)n * 2 * G + 2 * g + 1] / cnt - mean * mean);
-    rstd = rsqrtf(var + eps);
-#pragma unroll
-    for (int j = 0; j < 4; ++j) {
-      const float a0 = rstd * gam[2 * j], a1 = rstd * gam[2 * j + 1];
-      ah.v[j] = f2_pack(0.5f * a0, 0.5f * a1);
-      bh.v[j] = SILU ? f2_pack(0.5f * (bet[2 * j] - mean * a0), 0.5f * (bet[2 * j + 1] - mean * a1)) : f2_pack(0.f, 0.f);
-    }
-  };
-
-  auto pass1 = [&](int s) {
-    long long lo, hi; int n0;
-    slice(s, lo, hi, n0);
-    for (long long seg = lo; seg < hi;) {
-      const int img = (int)(seg / HW);
-      const long long seg_hi = min(hi, (long long)(img + 1) * HW);
-      const int n = n0 + img;
-      if (active) {
-        float mean, rstd; GnPair4 ah, bh, s0, s1;
-        coeffs(n, mean, rstd, ah, bh);
-#pragma unroll
-        for (int j = 0; j < 4; ++j) { s0.v[j] = f2_pack(0.f, 0.f); s1.v[j] = f2_pack(0.f, 0.f); }
-        const __nv_bfloat16* xb = x + (long long)n * HW * xps + cv * 8;
-        const __nv_bfloat16* db_ = dy + (long long)n * HW * dps + cv * 8;
-        const int p_lo = (int)(seg - (long long)img * HW), p_hi = (int)(seg_hi - (long long)img * HW);
-        for (int p0 = p_lo + r; p0 < p_hi; p0 += kBU * rows) {
-          uint4 xu[kBU], du[kBU];
-#pragma unroll
-          for (int k = 0; k < kBU; ++k) {
-            const int p = p0 + k * rows;
-            xu[k] = make_uint4(0, 0, 0, 0);
-            du[k] = make_uint4(0, 0, 0, 0);
-            if (p < p_hi) {
-              xu[k] = *reinterpret_cast<const uint4*>(xb + (long long)p * xps);
-              du[k] = *reinterpret_cast<const uint4*>(db_ + (long long)p * dps);
-            }
-          }
-#pragma unroll
-          for (int k = 0; k < kBU; ++k) {
-            const uint32_t xw[4] = {xu[k].x, xu[k].y, xu[k].z, xu[k].w};
-            const uint32_t dw[4] = {du[k].x, du[k].y, du[k].z, du[k].w};
-#pragma unroll
-            for (int j = 0; j < 4; ++j) {
-              const f32x2_t xv = f2_from_bf16x2(xw[j]);
-              const f32x2_t dz = gn_dz_pair<SILU, false>(xv, f2_from_bf16x2(dw[j]), ah.v[j], bh.v[j]);
-              s0.v[j] = f2_add(s0.v[j], dz);
-              s1.v[j] = f2_fma(dz, xv, s1.v[j]);
-            }
-          }
-        }
-#pragma unroll
-        for (int j = 0; j < 4; ++j) {
-          float l0, h0;
-          f2_unpack(s0.v[j], l0, h0);
-          part0[r * C + cv * 8 + 2 * j] = l0; part0[r * C + cv * 8 + 2 * j + 1] = h0;
-          f2_unpack(s1.v[j], l0, h0);
-          part1[r * C + cv * 8 + 2 * j] = l0; part1[r * C + cv * 8 + 2 * j + 1] = h0;
-        }
-      }
-      __syncthreads();
-      for (int c = tid; c < C; c += kNT) {
-        float t0 = 0.f, t1 = 0.f;
-        for (int rr = 0; rr < rows; ++rr) { t0 += part0[rr * C + c]; t1 += part1[rr * C + c]; }
-        atomicAdd(&ws[((long long)n * C + c) * 2], t0);
-        atomicAdd(&ws[((long long)n * C + c) * 2 + 1], t1);
-      }
-      __syncthreads();
-      seg = seg_hi;
-    }
-    __threadfence();
-    __syncthreads();
-    if (tid == 0) atomicAdd(&counters[s], 1u);
-  };
-
-  auto pass2 = [&](int s) {
-    if (tid == 0) {
-      while (ld_acquire_u32(&counters[s]) < nctas) __nanosleep(100);
-    }
-    __syncthreads();
-    long long lo, hi; int n0;
-    slice(s, lo, hi, n0);
-    for (long long seg = lo; seg < hi;) {
-      const int img = (int)(seg / HW);
-      const long long seg_hi = min(hi, (long long)(img + 1) * HW);
-      const int n = n0 + img;
-      if (tid < 2 * G) redg[tid] = 0.f;
-      __syncthreads();
-      for (int c = tid; c < C; c += kNT) {
-        const float S0 = __ldcg(&ws[((long long)n * C + c) * 2]), S1 = __ldcg(&ws[((long long)n * C + c) * 2 + 1]);
-        const int gc = c / cpg;
-        const float mg = stats[(long long)n * 2 * G + 2 * gc] / cnt;
-        const float vg = fmaxf(0.f, stats[(long long)n * 2 * G + 2 * gc + 1] / cnt - mg * mg);
-        const float rg = rsqrtf(vg + eps), ga = gamma[c];
-        atomicAdd(&redg[2 * gc], ga * S0);
-        atomicAdd(&redg[2 * gc + 1], ga * rg * (S1 - mg * S0));
-      }
-      __syncthreads();
-      if (active) {
-        float mean, rstd; GnPair4 ah, bh, cs;
-        coeffs(n, mean, rstd, ah, bh);
-        const float m1 = redg[2 * g] / cnt, m2 = redg[2 * g + 1] / cnt;
-        const float c2 = rstd * rstd * m2;
-        const float c3 = mean * c2 - rstd * m1;
-        const f32x2_t nc2 = f2_pack(-c2, -c2), c3p = f2_pack(c3, c3);
-#pragma unroll
-        for (int j = 0; j < 4; ++j) cs.v[j] = f2_pack(0.f, 0.f);
-        const __nv_bfloat16* xb = x + (long long)n * HW * xps + cv * 8;
-        const __nv_bfloat16* db_ = dy + (long long)n * HW * dps + cv * 8;
-        __nv_bfloat16* ob = dx + (long long)n * HW * dxps + cv * 8;
-        const __nv_bfloat16* ab_ = ACC ? acc + (long long)n * HW * accps + cv * 8 : nullptr;
-        const int p_lo = (int)(seg - (long long)img * HW), p_hi = (int)(seg_hi - (long long)img * HW);
-        for (int p0 = p_lo + r; p0 < p_hi; p0 += kBU * rows) {
-          uint4 xu[kBU], du[kBU], ou[kBU];
-#pragma unroll
-          for (int k = 0; k < kBU; ++k) {
-            const int p = p0 + k * rows;
-            xu[k] = make_uint4(0, 0, 0, 0);
-            du[k] = make_uint4(0, 0, 0, 0);
-            ou[k] = make_uint4(0, 0, 0, 0);
-            if (p < p_hi) {
-              xu[k] = *reinterpret_cast<const uint4*>(xb + (long long)p * xps);
-              du[k] = *reinterpret_cast<const uint4*>(db_ + (long long)p * dps);
-              if (ACC) ou[k] = *reinterpret_cast<const uint4*>(ab_ + (long long)p * accps);
-            }
-          }
-#pragma unroll
-          for (int k = 0; k < kBU; ++k) {
-            const int p = p0 + k * rows;
-            if (p < p_hi) {
-              const uint32_t xw[4] = {xu[k].x, xu[k].y, xu[k].z, xu[k].w};
-              const uint32_t dw[4] = {du[k].x, du[k].y, du[k].z, du[k].w};
-              const uint32_t ow[4] = {ou[k].x, ou[k].y, ou[k].z, ou[k].w};
-              uint32_t res[4];
-#pragma unroll
-              for (int j = 0; j < 4; ++j) {
-                const f32x2_t xv = f2_from_bf16x2(xw[j]);
-                const f32x2_t dz2 = gn_dz_pair<SILU, true>(xv, f2_from_bf16x2(dw[j]), ah.v[j], bh.v[j]);
-                f32x2_t v = f2_fma(dz2, ah.v[j], f2_fma(xv, nc2, c3p));
-                if (CS) cs.v[j] = f2_add(cs.v[j], v);
-                if (ACC) v = f2_add(v, f2_from_bf16x2(ow[j]));
-                res[j] = f2_to_bf16x2(v);
-              }
-              *reinterpret_cast<uint4*>(ob + (long long)p * dxps) = make_uint4(res[0], res[1], res[2], res[3]);
-            }
-          }
-        }
-        if (CS) {
-#pragma unroll
-          for (int j = 0; j < 4; ++j) {
-            float l0, h0;
-            f2_unpack(cs.v[j], l0, h0);
-            part0[r * C + cv * 8 + 2 * j] = l0;
-            part0[r * C + cv * 8 + 2 * j + 1] = h0;
-          }
-        }
-      }
-      if (CS) {
-        __syncthreads();
-        for (int c = tid; c < C; c += kNT) {
-          float v = 0.f;
-          for (int rr = 0; rr < rows; ++rr) v += part0[rr * C + c];
-          atomicAdd(&csum_img[(long long)n * C + c], v);
-        }
-      }
-      __syncthreads();
-      seg = seg_hi;
-    }
-  };
-
-  for (int s = 0; s < nstage; ++s) {
-    pass1(s);
-    if (s > 0) pass2(s - 1);
-  }
-  pass2(nstage - 1);
-}
-
-template <bool SILU, bool ACC, bool CS>
-int launch_bwd_pipe(const fdx_act* x, const fdx_act* dy, int groups, const float* stats, const float* gamma,
-                    const float* beta, float eps, float* ws, unsigned* counters, int max_stages,
-                    const fdx_act* dx, float* csum_img, const fdx_act* acc, cudaStream_t st) {
-  const int C = x->c, HW = x->h * x->w, N = x->n;
-  const size_t shm = sizeof(float) * (2 * (size_t)(kNT / (C / 8)) * C + 2 * groups);
-  static int occ = 0;
-  if (occ == 0) {
-    FDX_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, gn_bwd_pipe_kernel<SILU, ACC, CS>, kNT, 20 * 1024));
-    if (occ > 2) occ = 2;
-    if (occ < 1) occ = 1;
-  }
-  const int sms = fdx_num_sms();
-  const int grid = sms * occ;
-  // stage = whole images, ~24 MB of x + dy (two stages in flight), at least one image
-  const double img_bytes = 4.0 * HW * C;
-  int ips = (int)(24.0 * 1024 * 1024 / img_bytes);
-  if (ips < 1) ips = 1;
-  if (ips > N) ips = N;
-  while ((N + ips - 1) / ips > max_stages) ++ips;
-  const int nstage = (N + ips - 1) / ips;
-  FDX_CUDA(cudaMemsetAsync(counters, 0, sizeof(unsigned) * nstage, st));
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = dim3((unsigned)grid);
-  cfg.blockDim = dim3(kNT);
-  cfg.dynamicSmemBytes = shm;
-  cfg.stream = st;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeCooperative;     // all CTAs co-resident: the stage counters are spin-waited
-  attr[0].val.cooperative = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = 1;
-  FDX_CUDA(cudaLaunchKernelEx(&cfg, gn_bwd_pipe_kernel<SILU, ACC, CS>, (const __nv_bfloat16*)x->ptr,
-                              (long long)x->pix_stride, (const __nv_bfloat16*)dy->ptr, (long long)dy->pix_stride, N,
-                              HW, C, groups, ips, stats, gamma, beta, eps, ws, counters, (__nv_bfloat16*)dx->ptr,
-                              (long long)dx->pix_stride, csum_img, (const __nv_bfloat16*)(acc ? acc->ptr : nullptr),
-                              (long long)(acc ? acc->pix_stride : 0)));
-  fdx_count_launch();
-  return FDX_OK;
-}
-
-template <bool SILU, bool ACC, bool CS>
-int launch_bwd_cluster(int CL, size_t shm, const fdx_act* x, const fdx_act* dy, int groups, const float* stats,
-                       const float* gamma, const float* beta, float eps, float* ws, const fdx_act* dx,
-                       float* csum_img, const fdx_act* acc, cudaStream_t st) {
-  static bool attr_set = false;
-  if (!attr_set) {
-    FDX_CUDA(cudaFuncSetAttribute(gn_bwd_cluster_kernel<SILU, ACC, CS>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                  200 * 1024));
-    attr_set = true;
-  }
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = dim3((unsigned)(x->n * CL));
-  cfg.blockDim = dim3(kNT);
-  cfg.dynamicSmemBytes = shm;
-  cfg.stream = st;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeClusterDimension;
-  attr[0].val.clusterDim.x = (unsigned)CL;
-  attr[0].val.clusterDim.y = 1;
-  attr[0].val.clusterDim.z = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = 1;
-  FDX_CUDA(cudaLaunchKernelEx(&cfg, gn_bwd_cluster_kernel<SILU, ACC, CS>, (const __nv_bfloat16*)x->ptr,
-                              (long long)x->pix_stride, (const __nv_bfloat16*)dy->ptr, (long long)dy->pix_stride,
-                              x->h * x->w, x->c, groups, stats, gamma, beta, eps, ws, (__nv_bfloat16*)dx->ptr,
-                              (long long)dx->pix_stride, csum_img, (const __nv_bfloat16*)(acc ? acc->ptr : nullptr),
-                              (long long)(acc ? acc->pix_stride : 0)));
-  fdx_count_launch();
-  return FDX_OK;
-}
-
 // ---------------------------------------------------------------------------
 // RMSNorm over channels, one warp per pixel.
 // ---------------------------------------------------------------------------
@@ -1179,8 +584,8 @@ dim3 gn_grid(const fdx_act* x, int unroll, int resident) {
   const int HW = x->h * x->w;
   const int rows = kNT / (x->c / 8);
   int bx = (HW + rows * unroll - 1) / (rows * unroll);
-  static const int waves = getenv("FDX_GN_WAVES") ? atoi(getenv("FDX_GN_WAVES")) : 2;
-  int target = (waves * resident * 148) / x->n;
+  constexpr int kWaves = 2;
+  int target = (kWaves * resident * 148) / x->n;
   if (target < 1) target = 1;
   if (bx > target) bx = target;
   if (bx < 1) bx = 1;
@@ -1290,7 +695,6 @@ static int groupnorm_bwd_impl(const fdx_act* x, const fdx_act* dy, int groups, c
                               const float* gamma, const float* beta, float eps, int silu, float* ws,
                               float* dgamma, float* dbeta, const fdx_act* dx, const fdx_act* acc,
                               float* csum_img, float* csum_tot, void* stream) {
-  const int accumulate = acc != nullptr;
   int s = gn_check(x, groups, "groupnorm_bwd");
   if (s != FDX_OK) return s;
   FDX_REQUIRE(dy && dy->ptr && dx && dx->ptr && ws && dgamma && dbeta, "groupnorm_bwd: null tensor");
@@ -1300,122 +704,20 @@ static int groupnorm_bwd_impl(const fdx_act* x, const fdx_act* dy, int groups, c
   FDX_REQUIRE(!csum_tot || csum_img, "groupnorm_bwd: csum_tot needs csum_img");
   cudaStream_t st = (cudaStream_t)stream;
   const int N = x->n, C = x->c, HW = x->h * x->w;
-  float* sums = ws;                         // [N][C][2]
-  float* red = ws + 2LL * N * C;            // [N][G][2]
-  // One-launch cluster path (x and dy read from HBM once): images of >= 1024 pixels.  The cluster size sets
-  // both the parallelism per image and - with the shared-memory request that limits residency - how many
-  // images are in flight; their x + dy must stay well inside the L2.  FDX_GN_2PASS=1 keeps the two-pass path.
-  static const bool two_pass = [] {          // set and not "0" (the round-2 default sets it: flaxdiff_b200/_defaults.py)
-    const char* e = getenv("FDX_GN_2PASS");
-    return e && e[0] && e[0] != '0';
-  }();
-  const double img_bytes = 4.0 * HW * C;                      // x + dy of one image, bf16
-  int CL = 8;
-  while (CL > 1 && (HW / CL) < 4 * (kNT / (C / 8))) CL >>= 1;  // keep >= 4 row iterations per CTA
-  // images in flight with one CTA per SM = 148 / CL; beyond ~64 MB the second pass would miss in L2 anyway
-  const bool fits_l2 = (148.0 / CL) * img_bytes <= 64.0 * 1024 * 1024;
-  // FDX_GN_PIPE=1: the persistent pipelined kernel for the shapes the cluster path cannot take (large images);
-  // FDX_GN_PIPE=2: for every shape.  Its stage counters live behind `red` in the caller's workspace
-  // (2*N*groups floats >= the <= 2*N stages ever needed... capped to that many stages).
-  static const int pipe = getenv("FDX_GN_PIPE") ? atoi(getenv("FDX_GN_PIPE")) : 0;
-  if (!two_pass && pipe > 0 && (pipe > 1 || !(HW >= 1024 && fits_l2)) && (long long)N * HW >= 4096) {
-    FDX_CUDA(cudaMemsetAsync(sums, 0, sizeof(float) * 2 * N * C, st));
-    if (csum_img) FDX_CUDA(cudaMemsetAsync(csum_img, 0, sizeof(float) * N * C, st));
-    unsigned* counters = reinterpret_cast<unsigned*>(red);
-    const int max_stages = 2 * N * groups;
-    const int key = (silu ? 4 : 0) | (accumulate ? 2 : 0) | (csum_img ? 1 : 0);
-    int rc;
-#define FDX_GN_PP(S, A, CSF) rc = launch_bwd_pipe<S, A, CSF>(x, dy, groups, stats, gamma, beta, eps, sums, counters, max_stages, dx, csum_img, acc, st)
-    switch (key) {
-      case 0: FDX_GN_PP(false, false, false); break;
-      case 1: FDX_GN_PP(false, false, true); break;
-      case 2: FDX_GN_PP(false, true, false); break;
-      case 3: FDX_GN_PP(false, true, true); break;
-      case 4: FDX_GN_PP(true, false, false); break;
-      case 5: FDX_GN_PP(true, false, true); break;
-      case 6: FDX_GN_PP(true, true, false); break;
-      default: FDX_GN_PP(true, true, true); break;
-    }
-#undef FDX_GN_PP
-    if (rc != FDX_OK) return rc;
-    const int cb = (C + kFinC - 1) / kFinC;
-    gn_bwd_finalize_kernel<<<cb, 256, 0, st>>>(sums, stats, gamma, N, HW, C, groups, eps, cb, red, dgamma, dbeta);
-    FDX_LAUNCH_CHECK();
-    if (csum_tot) {
-      reduce_rows_kernel<<<(C + 31) / 32, 256, 0, st>>>(csum_img, N, C, csum_tot, 0);
-      FDX_LAUNCH_CHECK();
-    }
-    return FDX_OK;
-  }
-  if (!two_pass && HW >= 1024 && fits_l2) {
-    // CTAs per SM so that (148 * per_sm / CL) images * img_bytes <= 48 MB, at least 1
-    int per_sm = (int)((48.0 * 1024 * 1024 * CL) / (148.0 * img_bytes));
-    if (per_sm > 2) per_sm = 2;
-    if (per_sm < 1) per_sm = 1;
-    const size_t need = sizeof(float) * (2 * (size_t)(kNT / (C / 8)) * C + 2 * C + 2 * groups);
-    size_t shm = need;
-    const size_t force = per_sm == 1 ? 120 * 1024 : 0;       // > half of the SM's shared memory => one CTA / SM
-    if (shm < force) shm = force;
-    if (csum_img) FDX_CUDA(cudaMemsetAsync(csum_img, 0, sizeof(float) * N * C, st));
-    const int key = (silu ? 4 : 0) | (accumulate ? 2 : 0) | (csum_img ? 1 : 0);
-    int rc;
-#define FDX_GN_CL(S, A, CSF) rc = launch_bwd_cluster<S, A, CSF>(CL, shm, x, dy, groups, stats, gamma, beta, eps, sums, dx, csum_img, acc, st)
-    switch (key) {
-      case 0: FDX_GN_CL(false, false, false); break;
-      case 1: FDX_GN_CL(false, false, true); break;
-      case 2: FDX_GN_CL(false, true, false); break;
-      case 3: FDX_GN_CL(false, true, true); break;
-      case 4: FDX_GN_CL(true, false, false); break;
-      case 5: FDX_GN_CL(true, false, true); break;
-      case 6: FDX_GN_CL(true, true, false); break;
-      default: FDX_GN_CL(true, true, true); break;
-    }
-#undef FDX_GN_CL
-    if (rc != FDX_OK) return rc;
-    const int cb = (C + kFinC - 1) / kFinC;
-    gn_bwd_finalize_kernel<<<cb, 256, 0, st>>>(sums, stats, gamma, N, HW, C, groups, eps, cb, red, dgamma, dbeta);
-    FDX_LAUNCH_CHECK();
-    if (csum_tot) {
-      reduce_rows_kernel<<<(C + 31) / 32, 256, 0, st>>>(csum_img, N, C, csum_tot, 0);
-      FDX_LAUNCH_CHECK();
-    }
-    return FDX_OK;
-  }
-  // FDX_GN_FINALIZE=1: the round-1 sequence (sums workspace, finalize launch, reduce_rows launch)
-  static const bool separate_finalize = [] {
-    const char* e = getenv("FDX_GN_FINALIZE");
-    return e && e[0] && e[0] != '0';
-  }();
-  const bool merged = !separate_finalize;
-  if (merged) FDX_CUDA(cudaMemsetAsync(red, 0, sizeof(float) * 2 * N * groups, st));
-  else FDX_CUDA(cudaMemsetAsync(sums, 0, sizeof(float) * 2 * N * C, st));
-  const size_t shm = sizeof(float) * (2 * (size_t)(kNT / (C / 8)) * C + (merged ? 2 * C : 0));
-  float* red_arg = merged ? red : nullptr;
+  float* red = ws;                          // [N][G][2]: the per-group sums of pass 1
+  FDX_CUDA(cudaMemsetAsync(red, 0, sizeof(float) * 2 * N * groups, st));
+  const size_t shm = sizeof(float) * (2 * (size_t)(kNT / (C / 8)) * C + 2 * C);
   if (silu)
     gn_bwd_stats_kernel<true><<<gn_grid(x, kBU, 3), kNT, shm, st>>>(
         (const __nv_bfloat16*)x->ptr, x->pix_stride, (const __nv_bfloat16*)dy->ptr, dy->pix_stride, HW, C,
-        groups, stats, gamma, beta, eps, sums, red_arg, dgamma, dbeta, csum_img, csum_tot);
+        groups, stats, gamma, beta, eps, red, dgamma, dbeta, csum_img, csum_tot);
   else
     gn_bwd_stats_kernel<false><<<gn_grid(x, kBU, 3), kNT, shm, st>>>(
         (const __nv_bfloat16*)x->ptr, x->pix_stride, (const __nv_bfloat16*)dy->ptr, dy->pix_stride, HW, C,
-        groups, stats, gamma, beta, eps, sums, red_arg, dgamma, dbeta, csum_img, csum_tot);
+        groups, stats, gamma, beta, eps, red, dgamma, dbeta, csum_img, csum_tot);
   FDX_LAUNCH_CHECK();
-  if (merged) {
-    launch_bwd_apply(x, dy, groups, stats, red, gamma, beta, eps, silu, dx, acc, csum_img, st, csum_tot);
-    FDX_LAUNCH_CHECK();
-    return FDX_OK;
-  }
-  const int cb = (C + kFinC - 1) / kFinC, gb = (N * groups + 7) / 8;
-  gn_bwd_finalize_kernel<<<cb + gb, 256, 0, st>>>(sums, stats, gamma, N, HW, C, groups, eps, cb, red, dgamma,
-                                                   dbeta);
+  launch_bwd_apply(x, dy, groups, stats, red, gamma, beta, eps, silu, dx, acc, csum_img, st, csum_tot);
   FDX_LAUNCH_CHECK();
-  if (csum_img) FDX_CUDA(cudaMemsetAsync(csum_img, 0, sizeof(float) * N * C, st));
-  launch_bwd_apply(x, dy, groups, stats, red, gamma, beta, eps, silu, dx, acc, csum_img, st);
-  FDX_LAUNCH_CHECK();
-  if (csum_tot) {
-    reduce_rows_kernel<<<(C + 31) / 32, 256, 0, st>>>(csum_img, N, C, csum_tot, 0);
-    FDX_LAUNCH_CHECK();
-  }
   return FDX_OK;
 }
 
@@ -1450,50 +752,26 @@ int fdx_groupnorm_coeffs(const float* stats, const float* gamma, const float* be
 }
 
 static int groupnorm_bwd_dz_impl(const fdx_act* x, const fdx_act* dz, int groups, const float* stats,
-                                 const float* gamma, float eps, const float* ws_slots, int slots, float* ws,
+                                 const float* gamma, float eps, const float* ws_slots, int slots,
                                  float* dgamma, float* dbeta, const fdx_act* dx, const fdx_act* acc,
                                  float* csum_img, float* csum_tot, void* stream) {
   int s = gn_check(x, groups, "groupnorm_bwd_dz");
   if (s != FDX_OK) return s;
-  FDX_REQUIRE(dz && dz->ptr && dx && dx->ptr && ws && ws_slots && slots > 0 && dgamma && dbeta,
+  FDX_REQUIRE(dz && dz->ptr && dx && dx->ptr && ws_slots && slots > 0 && dgamma && dbeta,
               "groupnorm_bwd_dz: null tensor");
   FDX_REQUIRE(dz->c == x->c && dx->c == x->c && dz->n == x->n && dx->n == x->n && dz->h == x->h &&
                   dz->w == x->w && dx->h == x->h && dx->w == x->w,
               "groupnorm_bwd_dz: shape mismatch");
   FDX_REQUIRE(!csum_tot || csum_img, "groupnorm_bwd_dz: csum_tot needs csum_img");
   cudaStream_t st = (cudaStream_t)stream;
-  const int N = x->n, C = x->c, HW = x->h * x->w;
-  static const bool separate_finalize = [] {
-    const char* e = getenv("FDX_GN_FINALIZE");
-    return e && e[0] && e[0] != '0';
-  }();
-  if (!separate_finalize) {
-    // one launch: the apply kernel's prologue collapses the slots and derives the per-group constants
-    if (csum_img) FDX_CUDA(cudaMemsetAsync(csum_img, 0, sizeof(float) * N * C, st));
-    if (csum_tot) FDX_CUDA(cudaMemsetAsync(csum_tot, 0, sizeof(float) * C, st));
-    launch_bwd_apply(x, dz, groups, stats, nullptr, gamma, gamma, eps, 0, dx, acc, csum_img, st, csum_tot, ws_slots,
-                     slots, dgamma, dbeta);
-    FDX_LAUNCH_CHECK();
-    return FDX_OK;
-  }
-  float* sums = ws;                         // [N][C][2]
-  float* red = ws + 2LL * N * C;            // [N][G][2]
-  long long cg = ((long long)N * C + 255) / 256;
-  if (cg > 148 * 8) cg = 148 * 8;
-  gn_collapse_slots_kernel<<<(int)cg, 256, 0, st>>>(ws_slots, slots, N, C, sums);
-  FDX_LAUNCH_CHECK();
-  const int cb = (C + kFinC - 1) / kFinC, gb = (N * groups + 7) / 8;
-  gn_bwd_finalize_kernel<<<cb + gb, 256, 0, st>>>(sums, stats, gamma, N, HW, C, groups, eps, cb, red, dgamma,
-                                                   dbeta);
-  FDX_LAUNCH_CHECK();
+  const int N = x->n, C = x->c;
   if (csum_img) FDX_CUDA(cudaMemsetAsync(csum_img, 0, sizeof(float) * N * C, st));
-  // dz already carries silu'(z): the second pass is the activation-free one (beta is not read)
-  launch_bwd_apply(x, dz, groups, stats, red, gamma, gamma, eps, 0, dx, acc, csum_img, st);
+  if (csum_tot) FDX_CUDA(cudaMemsetAsync(csum_tot, 0, sizeof(float) * C, st));
+  // one launch: the apply kernel's prologue collapses the slots and derives the per-group constants; dz already
+  // carries silu'(z), so it is the activation-free second pass (beta is not read)
+  launch_bwd_apply(x, dz, groups, stats, nullptr, gamma, gamma, eps, 0, dx, acc, csum_img, st, csum_tot, ws_slots,
+                   slots, dgamma, dbeta);
   FDX_LAUNCH_CHECK();
-  if (csum_tot) {
-    reduce_rows_kernel<<<(C + 31) / 32, 256, 0, st>>>(csum_img, N, C, csum_tot, 0);
-    FDX_LAUNCH_CHECK();
-  }
   return FDX_OK;
 }
 
@@ -1501,7 +779,7 @@ int fdx_groupnorm_bwd_dz(const fdx_act* x, const fdx_act* dz, int groups, const 
                          const float* gamma, float eps, const float* ws_slots, int slots, float* ws,
                          float* dgamma, float* dbeta, const fdx_act* dx, int accumulate, float* csum_img,
                          float* csum_tot, void* stream) {
-  return groupnorm_bwd_dz_impl(x, dz, groups, stats, gamma, eps, ws_slots, slots, ws, dgamma, dbeta, dx,
+  return groupnorm_bwd_dz_impl(x, dz, groups, stats, gamma, eps, ws_slots, slots, dgamma, dbeta, dx,
                                accumulate ? dx : nullptr, csum_img, csum_tot, stream);
 }
 
@@ -1512,7 +790,7 @@ int fdx_groupnorm_bwd_dz_add(const fdx_act* x, const fdx_act* dz, int groups, co
   FDX_REQUIRE(addend && addend->ptr, "groupnorm_bwd_dz_add: null addend");
   FDX_REQUIRE(addend->c == x->c && addend->n == x->n && addend->h == x->h && addend->w == x->w,
               "groupnorm_bwd_dz_add: addend shape mismatch");
-  return groupnorm_bwd_dz_impl(x, dz, groups, stats, gamma, eps, ws_slots, slots, ws, dgamma, dbeta, dx, addend,
+  return groupnorm_bwd_dz_impl(x, dz, groups, stats, gamma, eps, ws_slots, slots, dgamma, dbeta, dx, addend,
                                csum_img, csum_tot, stream);
 }
 

@@ -55,7 +55,6 @@ def _attn_width(d: int) -> int:
 # engine got eight epilogue warps they beat the flat GEMM launch on the HBM-bound shapes
 # (profiles/layers_r02_res1x1.txt); FDX_RES1X1_GEMM=1 restores the flat launch.
 _RES1X1_GEMM = bool(os.environ.get("FDX_RES1X1_GEMM"))
-_GN_APPLY_V1 = bool(os.environ.get("FDX_GN_APPLY_V1"))
 
 class _SideStream:
     """Weight-gradient kernels have no consumer before the optimizer step, so the backward pass issues them
@@ -106,7 +105,7 @@ class Node:
     def colstats(self):
         """(workspace, channel offset) for a producer's epilogue, or None when the images are too small
         for the fused sums (the consumer then runs the statistics kernel)."""
-        if os.environ.get("FDX_NO_COLSTATS") or self.t.shape[1] * self.t.shape[2] < ops.COLSTATS_MIN_PIXELS:
+        if self.t.shape[1] * self.t.shape[2] < ops.COLSTATS_MIN_PIXELS:
             return None
         root = self.parent if self.parent is not None else self
         if root.cs is None:
@@ -125,11 +124,10 @@ class Node:
 
     def norm_apply(self, groups: int, gamma, beta, eps: float, silu: bool):
         """(GroupNorm(+SiLU) of this tensor, its statistics): ONE launch when the producers' epilogues left the
-        column sums (fdx_groupnorm_apply_cols), else statistics (from columns or by their own pass) + apply.
-        FDX_GN_APPLY_V1=1 keeps the separate stats_from_cols launch."""
+        column sums (fdx_groupnorm_apply_cols), else statistics (from columns or by their own pass) + apply."""
         done = all(k.cs_ok for k in self.kids) if self.kids else self.cs_ok
         root = self.parent if self.parent is not None else self
-        if done and root.cs is not None and groups <= 64 and not _GN_APPLY_V1:
+        if done and root.cs is not None and groups <= 64:
             return ops.groupnorm_apply_cols(self.t, groups, root.cs, self.coff, gamma, beta, eps, silu)
         st = self.stats(groups)
         return ops.groupnorm_apply(self.t, groups, st, gamma, beta, eps, silu), st
@@ -1032,14 +1030,7 @@ class Unet:
         dx, acc = want(xin)
         gn1 = (dh, W16[f"{name}/conv1/conv/kernel"], x, G, st1, W[f"{name}/{self._n1}/scale"],
                W[f"{name}/{self._n1}/bias"], RES_EPS, Gd[f"{name}/{self._n1}/scale"], Gd[f"{name}/{self._n1}/bias"], dx)
-        if os.environ.get("FDX_RES_BWD_V1"):        # round-1 order (GroupNorm backward, then the residual pass)
-            ops.conv_dgrad_groupnorm_bwd(*gn1, acc)
-            if cin != cout:
-                ops.gemm(GEMM_KK, dout, W16[kres + "kernel"].view(cin, cout), dx, M, cin, cout, dout.stride(2), cout,
-                         dx.stride(2), res=dx, r_ld=dx.stride(2))
-            else:
-                ops.act_add(dx, dout, dx)
-        elif cin != cout:
+        if cin != cout:
             if _RES1X1_GEMM:
                 ops.gemm(GEMM_KK, dout, W16[kres + "kernel"].view(cin, cout), dx, M, cin, cout, dout.stride(2), cout,
                          dx.stride(2), res=dx if acc else None, r_ld=dx.stride(2) if acc else 0)

@@ -183,7 +183,7 @@ def groupnorm_apply_cols(x, groups, cs: "ColStats", c0: int, gamma, beta, eps: f
 def groupnorm_bwd(x, dy, groups, stats, gamma, beta, eps, silu, dgamma, dbeta, dx,
                   accumulate: bool = False, csum_img=None, csum_tot=None, addend=None) -> torch.Tensor:
     """dx (+)= d/dx GroupNorm(+SiLU); `addend`: dx = d/dx + addend (another tensor of the same shape)."""
-    red = torch.empty(2 * x.shape[0] * (x.shape[-1] + groups), dtype=torch.float32, device=x.device)
+    red = torch.empty(2 * x.shape[0] * groups, dtype=torch.float32, device=x.device)
     if addend is not None:
         assert not accumulate
         check(load().fdx_groupnorm_bwd_add(ctypes.byref(act(x, "x")), ctypes.byref(act(dy, "dy")),
@@ -232,19 +232,18 @@ def conv3x3_dgrad_gn(dy: torch.Tensor, w_hwio: torch.Tensor, dz: torch.Tensor, x
 
 def groupnorm_bwd_dz(x, dz, groups, stats, gamma, eps, ws_slots, dgamma, dbeta, dx,
                      accumulate: bool = False, csum_img=None, csum_tot=None, addend=None) -> torch.Tensor:
-    red = torch.empty(2 * x.shape[0] * (x.shape[-1] + groups), dtype=torch.float32, device=x.device)
     if addend is not None:
         assert not accumulate, "groupnorm_bwd_dz: addend and accumulate are exclusive"
         check(load().fdx_groupnorm_bwd_dz_add(ctypes.byref(act(x, "x")), ctypes.byref(act(dz, "dz")),
                                               ctypes.c_int(groups), ptr(stats), ptr(gamma), ctypes.c_float(eps),
-                                              ptr(ws_slots), ctypes.c_int(ws_slots.shape[0]), ptr(red), ptr(dgamma),
+                                              ptr(ws_slots), ctypes.c_int(ws_slots.shape[0]), ptr(None), ptr(dgamma),
                                               ptr(dbeta), ctypes.byref(act(dx, "dx")),
                                               ctypes.byref(act(addend, "addend")), ptr(csum_img), ptr(csum_tot),
                                               stream_ptr()), "groupnorm_bwd_dz_add")
         return dx
     check(load().fdx_groupnorm_bwd_dz(ctypes.byref(act(x, "x")), ctypes.byref(act(dz, "dz")),
                                       ctypes.c_int(groups), ptr(stats), ptr(gamma), ctypes.c_float(eps),
-                                      ptr(ws_slots), ctypes.c_int(ws_slots.shape[0]), ptr(red), ptr(dgamma),
+                                      ptr(ws_slots), ctypes.c_int(ws_slots.shape[0]), ptr(None), ptr(dgamma),
                                       ptr(dbeta), ctypes.byref(act(dx, "dx")),
                                       ctypes.c_int(1 if accumulate else 0), ptr(csum_img), ptr(csum_tot),
                                       stream_ptr()), "groupnorm_bwd_dz")

@@ -469,7 +469,9 @@ class GeneralDiffusionTrainer:
         self._comm = get_comm() if (self.distributed_training and self.device.type == "cuda") else None
         nb = grad_buckets if grad_buckets is not None else int(os.environ.get("FDX_GRAD_BUCKETS", "4"))
         self._exchange = GradExchange(self._comm, self._gbuf, nb) if self._comm is not None else None
-        self._overlap = self._exchange is not None and os.environ.get("FDX_NO_DP_OVERLAP", "0") in ("", "0")
+        # one exchange after the backward unless FDX_NO_DP_OVERLAP is set to "0" (or ""): bucketed launches from the
+        # backward inside the training graph measured slower on 8 B200s (DESIGN 5)
+        self._overlap = self._exchange is not None and os.environ.get("FDX_NO_DP_OVERLAP") in ("", "0")
 
     # ------------------------------------------------------------------ state
     def generate_states(self, optimizer, rngs, existing_state=None, existing_best_state=None, model=None,

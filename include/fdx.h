@@ -140,7 +140,8 @@ int fdx_groupnorm_apply(const fdx_act* x, int groups, const float* stats, const 
 int fdx_groupnorm_apply_cols(const fdx_act* x, int groups, const float* cols, int slots, int ld, int c0,
                              const float* gamma, const float* beta, float eps, int silu, const fdx_act* y,
                              float* stats_out, void* stream);
-/* Backward of the pair above.  ws: f32 scratch of 2*N*C + 2*N*groups floats.  dgamma/dbeta ACCUMULATED.
+/* Backward of the pair above.  ws: f32 scratch of at least 2*N*groups floats (a larger buffer is fine; only
+ * the first 2*N*groups are used).  dgamma/dbeta ACCUMULATED.
  * csum_img [n][c] / csum_tot [c] (NULL allowed; csum_tot needs csum_img): column sums over pixels of the
  * dx this call produces, written (not accumulated) - the timestep row-vector and conv-bias gradients. */
 int fdx_groupnorm_bwd(const fdx_act* x, const fdx_act* dy, int groups, const float* stats,
@@ -160,7 +161,8 @@ int fdx_groupnorm_bwd_add(const fdx_act* x, const fdx_act* dy, int groups, const
  *                          dz = dgrad * silu'(a x + b) and ws_slots[slot][n][{0,1}][c] += (sum dz, sum dz*x);
  *                          zeroes ws_slots (slots*N*2*C floats) itself; FDX_ERR_UNSUPPORTED when an image
  *                          has fewer than 128 pixels (caller then uses the two-pass path)
- *   fdx_groupnorm_bwd_dz : second pass from dz; ws as in fdx_groupnorm_bwd. */
+ *   fdx_groupnorm_bwd_dz : second pass from dz, one launch; ws is not read (NULL allowed, kept for
+ *                          signature compatibility). */
 int fdx_groupnorm_coeffs(const float* stats, const float* gamma, const float* beta, int N, int HW, int C,
                          int groups, float eps, float* ab, void* stream);
 int fdx_conv3x3_dgrad_gn(const fdx_act* dy, const void* w_hwio, const fdx_act* dz, const fdx_act* x,

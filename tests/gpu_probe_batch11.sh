@@ -11,7 +11,7 @@ for v in "FDX_TC_BN_V1=1" "FDX_X=0"; do
 done
 echo "== attention old"; FDX_ATTN_NO_DUAL=1 FDX_ATTN_BWD_EWG1=1 timeout -s KILL 200 python tests/gpu_bench_attention.py 2>&1 | cut -c1-150
 echo "== attention new"; timeout -s KILL 200 python tests/gpu_bench_attention.py 2>&1 | cut -c1-150
-for v in "FDX_X=0" "FDX_GN_FINALIZE=1" "FDX_TC_BN_V1=1"; do
+for v in "FDX_X=0" "FDX_TC_BN_V1=1"; do
   echo "== bench c2 $v"
   env $v FDX_BENCH_CALLS=gpurun_out/calls_c2_$v.txt timeout -s KILL 200 python bench.py --workload c2 --no-cpu-baseline --steps 20 2>/dev/null | python -c "
 import sys,json

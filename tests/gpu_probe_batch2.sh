@@ -4,6 +4,4 @@ timeout -s KILL 300 python -m pytest tests/test_attention_gpu.py -q --tb=short 2
 echo "attention rc=${PIPESTATUS[0]}"
 timeout -s KILL 900 python -m pytest tests -m gpu -q --tb=short --deselect tests/test_attention_gpu.py --durations=12 2>&1 | tail -60
 echo "suite rc=${PIPESTATUS[0]}"
-FDX_GN_PIPE=2 timeout -s KILL 200 python -m pytest tests/test_kernels_gpu.py -q -k "groupnorm" --tb=short 2>&1 | tail -8
-FDX_GN_2PASS=1 timeout -s KILL 200 python -m pytest tests/test_kernels_gpu.py -q -k "groupnorm" --tb=short 2>&1 | tail -4
 bash tests/gpu_round2_ab.sh

@@ -1,7 +1,7 @@
 #!/bin/bash
 # round-2 batch 20: GroupNorm apply straight from the epilogue column sums (fdx_groupnorm_apply_cols)
 timeout -s KILL 900 python -m pytest tests/test_kernels_gpu.py tests/test_unet_gpu.py tests/test_baseline_shapes_gpu.py tests/test_train_gpu.py tests/test_samplers_gpu.py -q --tb=short -x 2>&1 | tail -5
-for v in "FDX_GN_APPLY_V1=1" "FDX_X=0" "FDX_GN_APPLY_V1=1" "FDX_X=1"; do
+for v in "FDX_X=0" "FDX_X=1"; do
   echo "== bench c2 $v"
   env $v timeout -s KILL 200 python bench.py --workload c2 --no-cpu-baseline --steps 20 2>/dev/null | python -c "
 import sys,json

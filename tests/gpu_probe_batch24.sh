@@ -1,6 +1,6 @@
 #!/bin/bash
-# zero-code A/Bs on the final library: GroupNorm grid waves, fused column statistics off
-for v in "FDX_X=0" "FDX_GN_WAVES=3" "FDX_GN_WAVES=4" "FDX_GN_WAVES=1" "FDX_NO_COLSTATS=1" "FDX_X=1"; do
+# run-to-run spread of the C2 line: the default configuration twice on one box
+for v in "FDX_X=0" "FDX_X=1"; do
   echo "== bench c2 $v"
   env $v timeout -s KILL 200 python bench.py --workload c2 --no-cpu-baseline --no-sample --steps 20 2>/dev/null | python -c "
 import sys,json

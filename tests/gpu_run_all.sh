@@ -8,6 +8,3 @@ echo "attention rc=$rc"; tail -25 gpurun_out/t_attn.log
 if [ $rc -ne 0 ]; then export FDX_ATTN_UNFUSED=1; echo "== running the rest with FDX_ATTN_UNFUSED=1"; fi
 timeout -s KILL 1200 python -m pytest tests -m gpu -q --deselect tests/test_attention_gpu.py 2>&1 | tail -60 > gpurun_out/t_all.log
 echo "suite rc=${PIPESTATUS[0]}"; tail -60 gpurun_out/t_all.log
-# opt-in GroupNorm-backward arrangements (read once per process): the persistent pipelined kernel and the two-pass one
-FDX_GN_PIPE=2 timeout -s KILL 300 python -m pytest tests/test_kernels_gpu.py -q -k "groupnorm" 2>&1 | tail -4
-FDX_GN_2PASS=1 timeout -s KILL 300 python -m pytest tests/test_kernels_gpu.py -q -k "groupnorm" 2>&1 | tail -4

@@ -49,12 +49,12 @@ dist.all_reduce(loss0); loss0 /= world
 
 res = {}
 for name, env, graph in (("overlap_graph", {"FDX_NO_DP_OVERLAP": "0"}, True), ("overlap_eager", {"FDX_NO_DP_OVERLAP": "0"}, False),
-                         ("single_call", {"FDX_NO_DP_OVERLAP": "1"}, True)):
+                         ("single_call", {"FDX_NO_DP_OVERLAP": "1"}, True), ("default", {}, True)):
     for k, v in env.items():
         os.environ[k] = v
     tr = make(use_cuda_graph=graph)
     assert tr._comm is not None and tr.world_size == world
-    assert tr._overlap == (env["FDX_NO_DP_OVERLAP"] == "0")
+    assert tr._overlap == (env.get("FDX_NO_DP_OVERLAP") == "0")   # unset: one exchange after the backward
     if graph:
         loss = tr._graphed_fwd_bwd(img, noise, t)
         loss = tr._graphed_fwd_bwd(img, noise, t)          # replay

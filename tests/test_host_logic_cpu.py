@@ -1,5 +1,9 @@
 """Host-side logic of the drop-in surface (schedulers / predictors coefficient algebra / sampler
 step sequences) against the NumPy oracle, on CPU tensors.  Integer timestep work is bit-exact."""
+import os
+import subprocess
+import sys
+
 import numpy as np
 import pytest
 import torch
@@ -175,3 +179,16 @@ def test_warmup_cosine_decay_schedule_values():
     assert abs(f(600) - mid) < 1e-10
     assert abs(f(1100) - 1e-5) < 1e-12 and abs(f(5000) - 1e-5) < 1e-12
     assert all(f(i) >= f(i + 1) for i in range(100, 1100, 37))
+
+
+def test_importing_the_package_sets_no_environment_switch():
+    """Kernel defaults live in the code that reads each switch: importing the package and the modules that read
+    FDX_* switches writes no FDX_* variable into os.environ, where every child process would inherit it."""
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    code = ("import os; before = dict(os.environ); "
+            "import flaxdiff_b200, flaxdiff_b200.ops, flaxdiff_b200.models.simple_unet, flaxdiff_b200.trainer; "
+            "print(sorted(k for k in os.environ if k.startswith('FDX_') and os.environ[k] != before.get(k)))")
+    env = {k: v for k, v in os.environ.items() if not k.startswith("FDX_")}
+    r = subprocess.run([sys.executable, "-c", code], cwd=root, env=env, capture_output=True, text=True, timeout=300)
+    assert r.returncode == 0, r.stderr[-2000:]
+    assert r.stdout.strip().splitlines()[-1] == "[]", r.stdout[-500:]

@@ -6,8 +6,6 @@ each is compared with the default arrangement AND with a plain fp32 torch convol
   FDX_NO_WGRAD9T=1  tap-pair arrangement of the nine-tap weight gradient
   FDX_WGRAD9_V1=1   round-1 nine-tap weight-gradient kernel instead of the kx-in-N one
   FDX_GN_FUSE=1     GroupNorm-backward first pass fused into the dgrad epilogue
-  FDX_GN_2PASS=0    one-launch CLUSTER GroupNorm backward (measured slower than the two-pass default; kept tested)
-  FDX_GN_PIPE=2     persistent software-pipelined GroupNorm backward (same)
 """
 import os
 
@@ -148,17 +146,3 @@ def test_groupnorm_backward_fused_into_dgrad(B, H, W, cin, cout):
     _conv_ref(Fnn.silu(xn).permute(0, 2, 3, 1), w).backward(dy.float())
     assert rel(outs[0][0], xr.grad) < 2e-2 and rel(outs[0][1], gr.grad) < 2e-2 and rel(outs[0][2], br.grad) < 2e-2
 
-
-@pytest.mark.parametrize("env_kv", [{"FDX_GN_2PASS": "0"}, {"FDX_GN_2PASS": "0", "FDX_GN_PIPE": "2"},
-                                    {"FDX_GN_FINALIZE": "1"}])
-def test_groupnorm_backward_single_launch_variants(env_kv):
-    """The cluster / pipelined GroupNorm-backward kernels and the round-1 separate-finalize sequence are selected
-    once per process: run the GroupNorm parity tests (all shapes, silu on/off, accumulate, column sums) in a
-    child process with the switch set."""
-    import subprocess
-    import sys
-    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    r = subprocess.run([sys.executable, "-m", "pytest", os.path.join(root, "tests", "test_kernels_gpu.py"), "-q",
-                        "-k", "groupnorm_fwd_bwd", "-p", "no:cacheprovider"], capture_output=True, text=True,
-                       env=dict(os.environ, **env_kv), timeout=600, cwd=root)
-    assert r.returncode == 0 and " passed" in r.stdout, r.stdout[-1500:] + r.stderr[-500:]
